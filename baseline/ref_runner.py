@@ -38,14 +38,14 @@ def main():
         print(json.dumps({"ok": False, "why": "baseline/_ref is empty (run __graft_entry__.build() where /root/reference exists)"}))
         return
     sys.path.insert(0, REF)
-    sys.path.append(ROOT)            # only for sketchedit_b200.synth (seeded checkpoints / inputs); `models` resolves to _ref
+    sys.path.append(ROOT)            # only for sketchedit_b200.synth and oracle.golden; `models` resolves to _ref
     from argparse import Namespace
 
-    import numpy as np
     import torch
     from models.editline2_model import EditLine2Model
     import models as ref_models
     assert os.path.realpath(ref_models.__file__).startswith(os.path.realpath(REF)), ref_models.__file__
+    from oracle.golden import Golden
     from sketchedit_b200 import synth
 
     opt = Namespace(gpu_ids=[], isTrain=False, isSkip=True, netG="deepfillc2", init_type="xavier", init_variance=0.02,
@@ -89,15 +89,14 @@ def main():
     out = {"ok": True, "kind": "reference", "images_per_s": args.batch / dt, "s_per_step": dt, "threads": threads, "cores": ncpu,
            "batch": args.batch, "size": args.size}
     if args.face:
-        z = np.load(os.path.join(ROOT, "tests", "golden", "face_602_256x256.npz"))
-        fimg = torch.from_numpy(z["image_u8"]).permute(2, 0, 1).float().div(255).sub(0.5).div(0.5)[None]
-        fsk = (torch.from_numpy(z["sketch_u8"]).float().div(255) > 0).float()[None, None]
+        g = Golden(os.path.join(ROOT, "tests", "golden", "face_602_256x256.npz"))
+        fimg, fsk = g.inputs()
         comp, _ = fwd(fimg, fsk)
         t0 = time.perf_counter()
         for _ in range(3):
             comp, _ = fwd(fimg, fsk)
         out["face_b1_s"] = (time.perf_counter() - t0) / 3
-        out["face_b1_max_abs_vs_golden"] = float((comp - torch.from_numpy(z["composed"])).abs().max())
+        out["face_b1_max_abs_vs_golden"] = g.maxdiff("composed", comp)
     print(json.dumps(out))
 
 

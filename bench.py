@@ -18,6 +18,12 @@ Prints ONE JSON line (rank 0):
   latency   batch-1 forward latency at 256x256 and 512x512 (N = 1, default workload only)
 `--impl reference` times the UNMODIFIED reference (baseline/_ref, staged by __graft_entry__.build()) on the host cores
 through baseline/ref_runner.py; if it was never staged, the CPU oracle port (kind "port").
+
+`--dump-outputs DIR` writes what the last timed step returned (composed [N,3,H,W] and mask [N,1,H,W], float32) as
+DIR/composed.npy and DIR/mask.npy, so that two builds can be compared output for output: inputs and weights are seeded, so
+the same arguments give the same inputs on every run. On several GPUs N is the all-gathered global batch. When the outputs
+exceed DUMP_BYTES, the same seeded sample of whole images is written for both. DIR/batch_index.txt lists, one per line, the
+batch index of each dumped image; image i of a batch has the inputs of image i % 8 (make_inputs repeats 8 base images).
 """
 import argparse
 import ctypes
@@ -36,6 +42,7 @@ if ROOT not in sys.path:
 import torch  # noqa: E402
 
 UNIT = "images/s"
+DUMP_BYTES = 64 * 10 ** 6
 
 
 def metric_name(size):
@@ -253,6 +260,24 @@ def load_traffic(workload_key):
     return (e["bytes_per_launch"], e["note"]) if e else (None, None)
 
 
+def dump_outputs(out_dir, outputs):
+    """outputs: {name: host tensor [N, C, H, W]} -> out_dir/<name>.npy (float32). Over DUMP_BYTES in all, every array keeps the
+    same seeded sample of its N images; out_dir/batch_index.txt lists the batch index of each image kept."""
+    import numpy as np
+    n = next(iter(outputs.values())).shape[0]
+    per_image = sum(t[0].numel() * 4 for t in outputs.values())
+    keep = min(n, DUMP_BYTES // per_image)
+    if keep == 0:
+        raise SystemExit("--dump-outputs: one image's outputs (%d bytes) exceed the %d-byte limit" % (per_image, DUMP_BYTES))
+    idx = np.arange(n) if keep == n else np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy()[idx].astype(np.float32))
+    with open(os.path.join(out_dir, "batch_index.txt"), "w") as f:
+        f.write("".join("%d\n" % i for i in idx))
+    return idx
+
+
 def write_class_table(path, rows, header):
     with open(path, "w") as f:
         f.write(header + "\n\n| us/step | launches/step | class | bound | achieved (algorithmic) | frac of bound |\n|---:|---:|---|---|---:|---:|\n")
@@ -303,8 +328,8 @@ def run_b200(args):
             slot = gather.next_slot()            # step i runs on NCCL's stream while step i+1 computes
             eng.inference_packed(img_d, sk_d, precision=prec, out=slot)
             gather.launch()
-        else:
-            eng.inference(img_d, sk_d, precision=prec)
+            return None
+        return eng.inference(img_d, sk_d, precision=prec)[:2]
 
     def barrier():
         if gather is not None:
@@ -314,7 +339,7 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     for _ in range(max(args.warmup, 3)):
-        step_device()
+        last = step_device()        # held like in the timed loop: both output allocations are cached before it
     barrier()
     launches_per_step = eng.launches()
 
@@ -326,11 +351,15 @@ def run_b200(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
     if gather is not None:
-        gather.wait()               # the last step's collective belongs to the region
+        last = parallel.unpack_outputs(gather.wait())      # the last step's collective belongs to the region
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:     # before the passes below reuse the gather ring
+        kept = dump_outputs(args.dump_outputs, {"composed": last[0].cpu(), "mask": last[1].cpu()})
+        print("bench: wrote the last timed step's outputs (%d of %d images) to %s" % (len(kept), last[0].shape[0], args.dump_outputs),
+              file=sys.stderr)
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -476,7 +505,13 @@ def main():
     ap.add_argument("--size", type=int, default=256, help="H = W of the synthetic inputs (256: CelebA-HQ configs, 512: Places config)")
     ap.add_argument("--classes-out", default=None, help="write the per-kernel-class roofline table (markdown) here")
     ap.add_argument("--no-latency", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32, a seeded sample of images beyond 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.batch is None:
         args.batch = 16 if args.size >= 512 else (128 if args.dtype == "bf16" else 32)
     if args.impl == "reference":

@@ -10,7 +10,7 @@ netM = MDGenerator, netG = DeepFillC2Generator), loads the seeded synthetic chec
 ``sketchedit_b200.synth`` through the reference's strict ``load_state_dict`` and calls the
 reference forward ``model(data, mode='inference')`` (reference models/editline2_model.py:107-133)
 plus forward hooks on a few inner modules. Nothing from the reference is copied into the
-repo: only the numeric inputs/outputs are stored.
+repo: only the numeric inputs/outputs are stored, in the format of ``oracle/golden.py``.
 """
 import argparse
 import os
@@ -65,6 +65,7 @@ def main():
     ap.add_argument("--only", default=None, help="comma-separated case names (default: all)")
     args = ap.parse_args()
     sys.path.insert(0, ROOT)
+    from oracle import golden
     from sketchedit_b200 import synth
     torch.set_num_threads(8)
     WM, WG = synth.synth_state_dict("M"), synth.synth_state_dict("G")
@@ -119,16 +120,13 @@ def main():
         for k, v in taps.items():
             out["tap:" + k] = v.numpy()
         if "u8" in case:
-            out["image_u8"], out["sketch_u8"] = case["u8"]
-            # keep the big cases small: only end-to-end tensors (+ what the case asks for)
-            for k in list(out):
-                if k not in ("composed", "mask", "image_u8", "sketch_u8") + tuple(case["keep"]):
-                    del out[k]
+            inputs = dict(image_u8=case["u8"][0], sketch_u8=case["u8"][1])
+            # the real-image cases: only end-to-end tensors (+ what the case asks for)
+            out = {k: v for k, v in out.items() if k in ("composed", "mask") + tuple(case["keep"])}
         else:
-            out["image"], out["sketch"] = image.numpy(), sketch.numpy()
-        out["flags"] = np.array(repr(sorted(case["flags"].items())))
+            inputs = dict(image=image.numpy(), sketch=sketch.numpy())
         path = os.path.join(args.out, name + ".npz")
-        np.savez_compressed(path, **out)
+        golden.save(path, inputs, out, case["flags"])
         print("wrote %s  (%.1f KB)  mask-on %.3f" % (path, os.path.getsize(path) / 1024,
                                                       float((mask > 0.5).float().mean())))
 

@@ -14,19 +14,12 @@ import pytest
 import torch
 
 from oracle import sketchedit_oracle as O
+from oracle.golden import Golden
 from sketchedit_b200 import synth
 from tests.util_parity import engine, maxdiff, weights
 
 pytestmark = pytest.mark.gpu
 TOL = {"fp32": 1e-3, "fp32_direct": 1e-3, "bf16": 1e-2}   # "fp32": split-half tensor-core arithmetic, "fp32_direct": CUDA cores
-
-
-def _golden_inputs(z):
-    if "image" in z:
-        return torch.from_numpy(z["image"]), torch.from_numpy(z["sketch"])
-    image = torch.from_numpy(z["image_u8"]).permute(2, 0, 1).float().div(255).sub(0.5).div(0.5)[None]
-    sketch = (torch.from_numpy(z["sketch_u8"]).float().div(255) > 0).float()[None, None]
-    return image, sketch
 
 
 @pytest.mark.parametrize("prec", ["fp32", "fp32_direct", "bf16"])
@@ -75,26 +68,24 @@ def test_inference_vs_oracle(prec, shape):
 def test_fp32_path_matches_reference_golden(name, golden_dir, prec):
     """fp32 paths (tensor-core split-half arithmetic and the CUDA-core cross-check) vs outputs of the unmodified reference
     (tests/golden, oracle/make_golden.py)."""
-    z = np.load(os.path.join(golden_dir, name + ".npz"))
-    image, sketch = _golden_inputs(z)
-    flags = dict(eval(str(z["flags"])))
-    eng = engine(**flags)
+    g = Golden(os.path.join(golden_dir, name + ".npz"))
+    image, sketch = g.inputs()
+    eng = engine(**g.flags)
     composed, mask, ex = eng.inference(image.cuda(), sketch.cuda(), precision=prec, want=("fine", "mask_bin"))
-    ref_bin = (torch.from_numpy(z["mask"]) > 0.5).float()
-    assert int((ex["mask_bin"].cpu() != ref_bin).sum()) == 0
-    assert maxdiff(mask.cpu(), torch.from_numpy(z["mask"])) <= 1e-3
-    if "fine" in z:
-        assert maxdiff(ex["fine"].cpu(), torch.from_numpy(z["fine"])) <= 1e-3
-    assert maxdiff(composed.cpu(), torch.from_numpy(z["composed"])) <= 1e-3
+    assert int((ex["mask_bin"].cpu() != g.mask_bin()).sum()) == 0
+    assert g.maxdiff("mask", mask) <= 1e-3
+    if "fine" in g:
+        assert g.maxdiff("fine", ex["fine"]) <= 1e-3
+    assert g.maxdiff("composed", composed) <= 1e-3
 
 
 def test_bf16_face_config(golden_dir):
     """BASELINE.json config: 256x256 face + sketch, bf16 tensor-core path, 1e-2 vs the fp32 reference."""
     WM, WG = weights()
-    z = np.load(os.path.join(golden_dir, "face_602_256x256.npz"))
-    image, sketch = _golden_inputs(z)
+    g = Golden(os.path.join(golden_dir, "face_602_256x256.npz"))
+    image, sketch = g.inputs()
     composed, mask, ex = engine().inference(image.cuda(), sketch.cuda(), precision="bf16", want=("mask_bin",))
-    assert maxdiff(mask.cpu(), torch.from_numpy(z["mask"])) <= 1e-2
+    assert g.maxdiff("mask", mask) <= 1e-2
     ours_bin = ex["mask_bin"].cpu()
     ref = O.inference(WM, WG, image, sketch, mask_bin_override=ours_bin)
     assert maxdiff(composed.cpu(), ref["composed"]) <= 1e-2

@@ -1,27 +1,16 @@
-"""Pin the CPU oracle against outputs of the UNMODIFIED reference (tests/golden/*.npz,
-made by oracle/make_golden.py from /root/reference in the build container)."""
+"""Pin the CPU oracle against outputs of the UNMODIFIED reference (tests/golden/*.npz, made by oracle/make_golden.py
+from the original project; format: oracle/golden.py)."""
 import glob
 import os
 
-import numpy as np
 import pytest
 import torch
 
 from oracle import sketchedit_oracle as O
+from oracle.golden import Golden
 from sketchedit_b200 import synth
 
 TOL = 2e-5   # fp32 vs fp32, different op order (attention form vs grouped conv)
-
-
-def _load(path):
-    z = np.load(path)
-    if "image" in z:
-        image, sketch = torch.from_numpy(z["image"]), torch.from_numpy(z["sketch"])
-    else:   # uint8 inputs: reference data/testimage_dataset.py:89-103 preprocessing
-        image = torch.from_numpy(z["image_u8"]).permute(2, 0, 1).float().div(255).sub(0.5).div(0.5)[None]
-        sketch = (torch.from_numpy(z["sketch_u8"]).float().div(255) > 0).float()[None, None]
-    flags = dict(eval(str(z["flags"])))
-    return z, image, sketch, flags
 
 
 @pytest.fixture(scope="module")
@@ -33,21 +22,20 @@ def weights():
                                         glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz"))))
 def test_oracle_matches_reference(name, weights, golden_dir):
     WM, WG = weights
-    z, image, sketch, flags = _load(os.path.join(golden_dir, name + ".npz"))
+    g = Golden(os.path.join(golden_dir, name + ".npz"))
+    image, sketch = g.inputs()
     taps = {}
-    r = O.inference(WM, WG, image, sketch, taps=taps, **flags)
+    r = O.inference(WM, WG, image, sketch, taps=taps, **g.flags)
     # the binarised mask must agree exactly (otherwise nothing downstream is comparable)
-    ref_bin = torch.from_numpy(z["mask"]) > 0.5
-    assert int((ref_bin != (r["mask_bin"] > 0.5)).sum()) == 0
+    assert int((g.mask_bin() != (r["mask_bin"] > 0.5).float()).sum()) == 0
     for key in ("composed", "mask", "coarse", "fine"):
-        if key in z:
-            d = float((r[key] - torch.from_numpy(z[key])).abs().max())
+        if key in g:
+            d = g.maxdiff(key, r[key])
             assert d <= TOL, (name, key, d)
-    for key in z.files:
+    for key in g.keys:
         if key.startswith("tap:"):
-            ours = taps[key[4:]]
-            d = float((ours - torch.from_numpy(z[key])).abs().max())
-            scale = max(1.0, float(torch.from_numpy(z[key]).abs().max()))
+            d = g.maxdiff(key, taps[key[4:]])
+            scale = max(1.0, g.absmax(key))
             assert d <= TOL * scale * 4, (name, key, d)
 
 
