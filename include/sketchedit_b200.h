@@ -104,6 +104,22 @@ int se_contextual_attention_forward(const float* feat, const float* mask_s, int 
 int se_outputs_to_uint8(const float* composed, const float* mask, int B, int H, int W, unsigned char* bgr_hwc,
                         unsigned char* mask_u8, void* stream);
 
+/* ---- Pillow's Image.resize((w, h)) with its default filter (BICUBIC) on uint8 HWC images, bit for bit: the resizes of the
+ *      reference's demo.py:45,49,68 (to a multiple of 8 and back) on the device. Uses no model.
+ * A ragged batch of B images with C = 1 or 3 channels: image i is src_hw[2i] x src_hw[2i+1] (height, width) at byte offset
+ * src_off[i] from src and becomes dst_hw[2i] x dst_hw[2i+1] at byte offset dst_off[i] from dst. src_off, src_hw, dst_off and
+ * dst_hw are HOST arrays; src and dst are device pointers (the images must not overlap their outputs). One launch per pass
+ * (horizontal, then vertical) covers the batch. flags: SE_RESIZE_REVERSE_CHANNELS writes the channels reversed (BGR <-> RGB),
+ * images of unchanged size included (those are copied, as Pillow does). The coefficient tables of every (in, out) pair are
+ * built on the host the first time the pair is seen on a device and stay cached there. */
+enum { SE_RESIZE_REVERSE_CHANNELS = 1 };
+int se_resize_u8(const unsigned char* src, const long long* src_off, const int* src_hw, int B, int C, unsigned char* dst,
+                 const long long* dst_off, const int* dst_hw, int flags, void* stream);
+/* Host only (no device needed): the coefficient tables of one in -> out pass of se_resize_u8. Returns ksize, the weights per
+ * output index, or -1 on error. bounds [out][2] = (first source index, tap count); weights [out][ksize] int32 in 22-bit fixed
+ * point, zero past the tap count. They are written only if bounds and weights are non-NULL and cap >= out * ksize. */
+int se_resize_coeffs(int in, int out, int* bounds, int* weights, int cap);
+
 /* ---- introspection for bench.py */
 /* number of kernels this library launched during the most recent forward-type call on this thread */
 int se_last_launch_count(void);

@@ -39,6 +39,8 @@ SIGNATURES = {
     "se_contextual_attention_forward": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_int, _c_void_p,
                                                  _c_void_p, _c_void_p]),
     "se_outputs_to_uint8": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p, _c_void_p, _c_void_p]),
+    "se_resize_u8": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_void_p, _c_void_p, _c_void_p, _c_int, _c_void_p]),
+    "se_resize_coeffs": (_c_int, [_c_int, _c_int, _c_void_p, _c_void_p, _c_int]),
     "se_last_launch_count": (_c_int, []),
     "se_workspace_bytes": (ctypes.c_longlong, [_c_void_p]),
     "se_timing_enable": (_c_int, [_c_int]),
@@ -78,4 +80,5 @@ def check(rc):
 
 # "fp32": fp32-parity arithmetic on the tensor cores (split-half fp16, SE_PREC_FP32_TC); "fp32_direct": the fp32 CUDA-core kernels
 PREC = {"bf16": 0, "fp32": 3, "fp32_direct": 1, "bf16_direct": 2}
+RESIZE_REVERSE_CHANNELS = 1   # SE_RESIZE_REVERSE_CHANNELS
 OPT = {"use_cam": 0, "pool_avg": 1, "no_mask_cc": 2, "no_mask_coarse": 3, "joint_train_inp": 4}

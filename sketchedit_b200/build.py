@@ -13,9 +13,11 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsketchedit_b200.so")
-SOURCES = ["se_engine.cu", "se_conv_c8.cu", "se_cam.cu", "se_conv_direct.cu", "se_misc.cu", "se_split.cu", "se_gemm_split.cu"]
+SOURCES = ["se_engine.cu", "se_conv_c8.cu", "se_cam.cu", "se_conv_direct.cu", "se_misc.cu", "se_split.cu", "se_gemm_split.cu", "se_resize.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
+# the resize coefficient tables must round exactly like Pillow's: no fused multiply-adds in their host code
+SOURCE_FLAGS = {"se_resize.cu": ["-Xcompiler", "-ffp-contract=off"]}
 
 
 def _nvcc():
@@ -44,7 +46,7 @@ def build(force=False, verbose=True):
     for src in SOURCES:
         obj = os.path.join(HERE, "build", src.replace(".cu", ".o"))
         objs.append(obj)
-        cmd = [nvcc] + flags + ["-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc] + flags + SOURCE_FLAGS.get(src, []) + ["-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             print(" ".join(cmd), flush=True)
         procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))

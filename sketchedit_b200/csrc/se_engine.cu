@@ -23,6 +23,7 @@
 #include "se_gemm_split.h"
 #include "se_conv_tc.h"
 #include "se_misc.h"
+#include "se_resize.h"
 
 namespace se {
 
@@ -1638,6 +1639,96 @@ int se_outputs_to_uint8(const float* composed, const float* mask, int B, int H, 
                         void* stream) {
   SE_REQUIRE(composed && bgr_hwc && (mask || !mask_u8), "null tensor");
   return to_uint8(composed, mask, bgr_hwc, mask_u8, B, H, W, (cudaStream_t)stream);
+}
+
+int se_resize_u8(const unsigned char* src, const long long* src_off, const int* src_hw, int B, int C, unsigned char* dst,
+                 const long long* dst_off, const int* dst_hw, int flags, void* stream) {
+  SE_REQUIRE(src && src_off && src_hw && dst && dst_off && dst_hw, "null argument");
+  SE_REQUIRE(B >= 1 && B <= 65535, "B must be in [1, 65535] (one grid row per image)");
+  SE_REQUIRE(C == 1 || C == 3, "C must be 1 or 3");
+  SE_REQUIRE((flags & ~SE_RESIZE_REVERSE_CHANNELS) == 0, "unknown flag");
+  for (int i = 0; i < B; ++i) {
+    const long long hi = src_hw[2 * i], wi = src_hw[2 * i + 1], ho = dst_hw[2 * i], wo = dst_hw[2 * i + 1];
+    SE_REQUIRE(hi >= 1 && wi >= 1 && ho >= 1 && wo >= 1, "image " + std::to_string(i) + ": sizes must be positive");
+    SE_REQUIRE(std::max(hi, ho) * std::max(wi, wo) * C < (1LL << 31), "image " + std::to_string(i) + ": too large");
+    SE_REQUIRE(src_off[i] >= 0 && dst_off[i] >= 0, "image " + std::to_string(i) + ": negative offset");
+  }
+  // arena owner of the model-less operator, one per device (like se_contextual_attention_forward's)
+  static std::mutex holders_mu;
+  static std::map<int, se_model*> holders;
+  int dev = -1;
+  SE_CUDA_OK(cudaGetDevice(&dev));
+  se_model* holder;
+  {
+    std::lock_guard<std::mutex> lk(holders_mu);
+    se_model*& h = holders[dev];
+    if (!h) { h = new se_model(); h->finalized = true; }
+    holder = h;
+  }
+  const int rev = (flags & SE_RESIZE_REVERSE_CHANNELS) ? 1 : 0;
+  return with_arena(holder, SE_PREC_BF16_TC, B, (cudaStream_t)stream, [&](Ctx& c) -> int {
+    // scratch: the jobs of both passes, then the uint8 intermediate of every image whose width AND height change
+    std::vector<size_t> tmp_off(B, 0);
+    size_t tmp_bytes = 0;
+    for (int i = 0; i < B; ++i)
+      if (src_hw[2 * i] != dst_hw[2 * i] && src_hw[2 * i + 1] != dst_hw[2 * i + 1]) {
+        tmp_off[i] = tmp_bytes;
+        tmp_bytes += ((size_t)src_hw[2 * i] * dst_hw[2 * i + 1] * C + 255) / 256 * 256;
+      }
+    Buf jb = c.get((size_t)2 * B * sizeof(ResizeJob));
+    Buf tmp = c.get(tmp_bytes);
+    if (!c.dry) {
+      std::vector<ResizeJob> hj, vj;
+      long long hmax = 0, vmax = 0;
+      for (int i = 0; i < B; ++i) {
+        const int hi = src_hw[2 * i], wi = src_hw[2 * i + 1], ho = dst_hw[2 * i], wo = dst_hw[2 * i + 1];
+        const unsigned char* in = src + src_off[i];
+        unsigned char* out = dst + dst_off[i];
+        if (wi != wo || hi == ho) {   // horizontal pass, or the copy of an unchanged size
+          ResizeJob j{in, hi != ho ? (unsigned char*)tmp.p + tmp_off[i] : out, nullptr, nullptr, 0, wi, hi, wo, hi != ho ? 0 : rev};
+          if (wi != wo) {
+            ResizeTable t;
+            int r = resize_table(wi, wo, c.stream, &t);
+            if (r) return r;
+            j.bounds = t.bounds; j.weights = t.weights; j.ksize = t.ksize;
+          }
+          hj.push_back(j);
+          hmax = std::max(hmax, (long long)hi * wo);
+          if (hi != ho) in = j.out;
+        }
+        if (hi != ho) {
+          ResizeTable t;
+          int r = resize_table(hi, ho, c.stream, &t);
+          if (r) return r;
+          vj.push_back(ResizeJob{in, out, t.bounds, t.weights, t.ksize, wo, ho, wo, rev});
+          vmax = std::max(vmax, (long long)ho * wo);
+        }
+      }
+      const size_t nh = hj.size();
+      hj.insert(hj.end(), vj.begin(), vj.end());
+      SE_CUDA_OK(cudaMemcpyAsync(jb.p, hj.data(), hj.size() * sizeof(ResizeJob), cudaMemcpyHostToDevice, c.stream));
+      const ResizeJob* jobs = (const ResizeJob*)jb.p;
+      if (nh) CK(resize_pass(jobs, (int)nh, hmax, C, 0, c.stream));
+      if (!vj.empty()) CK(resize_pass(jobs + nh, (int)vj.size(), vmax, C, 1, c.stream));
+    }
+    c.put(tmp);
+    c.put(jb);
+    return 0;
+  });
+}
+
+int se_resize_coeffs(int in, int out, int* bounds, int* weights, int cap) {
+  if (in < 1 || out < 1) {
+    se::set_error("se_resize_coeffs: sizes must be positive");
+    return -1;
+  }
+  std::vector<int> b, w;
+  const int ksize = resize_coeffs(in, out, b, w);
+  if (bounds && weights && (long long)cap >= (long long)w.size()) {
+    memcpy(bounds, b.data(), b.size() * sizeof(int));
+    memcpy(weights, w.data(), w.size() * sizeof(int));
+  }
+  return ksize;
 }
 
 int se_last_launch_count(void) { return se::g_launches; }

@@ -7,7 +7,9 @@ exposes the reference's call surface for the generator forward pass with CUDA te
 PyTorch is plumbing here (device memory + current stream); all compute is in libsketchedit_b200.so.
 """
 import ctypes
+from itertools import accumulate
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -39,6 +41,77 @@ def _chk_out(t, shape, name):
 
 def _f32(*shape, like):
     return torch.empty(*shape, device=like.device, dtype=torch.float32)
+
+
+def _chk_u8(t, name):
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.uint8 and t.is_contiguous()):
+        raise _lib.SketchEditB200Error("%s must be a contiguous CUDA uint8 tensor" % name)
+    return t
+
+
+def resize_u8(src, dst_hw, src_hw=None, channels=None, src_offsets=None, out=None, out_offsets=None, reverse_channels=False):
+    """Pillow's ``Image.resize((w, h))`` with its default filter (BICUBIC) on the device, bit for bit (se_resize_u8): a ragged
+    batch of uint8 HWC images, image i to size ``dst_hw[i] = (h, w)``, one launch per pass. Uses no model.
+
+    * ``src`` a list of CUDA uint8 tensors [H,W,C] (C = 1 or 3) or [H,W]: returns a list of tensors [h,w,C] (or [h,w]), views of
+      one new buffer.
+    * ``src`` a packed CUDA uint8 buffer with ``src_hw`` (one (H, W) per image) and ``channels``: the images lie back to back, or at
+      byte offsets ``src_offsets``. Returns the flat output buffer with the results back to back, or writes them into ``out``
+      at byte offsets ``out_offsets`` and returns ``out``.
+
+    ``reverse_channels`` writes the channels reversed (RGB <-> BGR)."""
+    listed = isinstance(src, (list, tuple))
+    if listed:
+        if not src:
+            return []
+        for i, t in enumerate(src):
+            _chk_u8(t, "src[%d]" % i)
+            if t.dim() not in (2, 3) or t.device != src[0].device:
+                raise _lib.SketchEditB200Error("src[%d] must be [H,W] or [H,W,C] on %s" % (i, src[0].device))
+        shapes = {t.shape[2:] for t in src}
+        if len(shapes) != 1:
+            raise _lib.SketchEditB200Error("all images of a batch need the same channel count")
+        channels = src[0].shape[2] if src[0].dim() == 3 else 1
+        src_hw = [tuple(t.shape[:2]) for t in src]
+        base = min(t.data_ptr() for t in src)
+        src_offsets = [t.data_ptr() - base for t in src]
+        device = src[0].device
+    else:
+        _chk_u8(src, "src")
+        if src_hw is None or channels is None:
+            raise _lib.SketchEditB200Error("a packed src needs src_hw and channels")
+        base, device = src.data_ptr(), src.device
+    B, C = len(src_hw), int(channels)
+    if len(dst_hw) != B:
+        raise _lib.SketchEditB200Error("dst_hw has %d sizes for %d images" % (len(dst_hw), B))
+    if min(min(hw) for hw in list(src_hw) + list(dst_hw)) < 1:
+        raise _lib.SketchEditB200Error("image sizes must be positive")
+    src_n = [int(h) * int(w) * C for h, w in src_hw]
+    dst_n = [int(h) * int(w) * C for h, w in dst_hw]
+    if src_offsets is None:
+        src_offsets = [0] + list(accumulate(src_n))[:-1]
+    if not listed and any(o < 0 or o + n > src.numel() for o, n in zip(src_offsets, src_n)):
+        raise _lib.SketchEditB200Error("an image lies outside src")
+    if out is None:
+        if out_offsets is not None:
+            raise _lib.SketchEditB200Error("out_offsets needs out")
+        out = torch.empty(sum(dst_n), device=device, dtype=torch.uint8)
+    elif _chk_u8(out, "out").device != device:
+        raise _lib.SketchEditB200Error("out must be on %s" % device)
+    if out_offsets is None:
+        out_offsets = [0] + list(accumulate(dst_n))[:-1]
+    if any(o < 0 or o + n > out.numel() for o, n in zip(out_offsets, dst_n)):
+        raise _lib.SketchEditB200Error("an image lies outside out")
+    i64 = lambda v: np.ascontiguousarray(v, dtype=np.int64)
+    i32 = lambda v: np.ascontiguousarray(np.asarray(v, dtype=np.int64).reshape(B, 2), dtype=np.int32)
+    so, shw, do, dhw = i64(src_offsets), i32(src_hw), i64(out_offsets), i32(dst_hw)
+    with torch.cuda.device(device):
+        _lib.check(_lib.load().se_resize_u8(ctypes.c_void_p(base), so.ctypes.data, shw.ctypes.data, B, C, _ptr(out), do.ctypes.data,
+                                            dhw.ctypes.data, _lib.RESIZE_REVERSE_CHANNELS if reverse_channels else 0, _stream()))
+    if not listed:
+        return out
+    return [out[o:o + n].view(h, w, C) if src[i].dim() == 3 else out[o:o + n].view(h, w)
+            for i, (o, n, (h, w)) in enumerate(zip(out_offsets, dst_n, dst_hw))]
 
 
 class Engine:
@@ -166,6 +239,9 @@ class Engine:
         _lib.check(self.lib.se_forward_inference_u8(self.h, _ptr(image_u8), _ptr(sketch_u8), B, H, W, _lib.PREC[precision], _ptr(bgr), _ptr(mk),
                                                     _stream()))
         return bgr, mk
+
+    # the model-less device resize, next to the forward it brackets in serving (and replaceable there by a test double)
+    resize_u8 = staticmethod(resize_u8)
 
     def netM(self, x, guide, precision="bf16", want_image=True):
         x, guide = _chk_in(x), _chk_in(guide)

@@ -4,7 +4,8 @@ The reference's demo handles one request per Flask thread (``app.run(threaded=Tr
 batch-1 forward. Here concurrent requests are BATCHED: ``RequestBatcher`` collects the requests that arrive within a short
 window, groups them by input size and runs each group as one forward (``Engine.inference_u8``: the codecs of
 demo.py:52-53,64-66 run on the device); ``DemoProcessor.process_image`` is the reference's ``process_image`` around it
-(floor the size to a multiple of 8, PIL resize in, forward, PIL resize back).
+(floor the size to a multiple of 8, PIL resize in, forward, PIL resize back). With ``resize="device"`` the three resizes run
+on the device too (``engine.resize_u8``, bit for bit Pillow's), so one batch holds every raw size that floors to its key.
 
     proc = DemoProcessor(models.create_model(opt), max_batch=16, max_wait_ms=2.0)
     result_pil = proc.process_image(image_pil, mask_pil)       # callable from any number of threads
@@ -122,13 +123,17 @@ class DemoProcessor:
     ``static/results/<name>``, and concurrent calls share forwards. ``precision``: 'bf16' | 'fp32' | 'fp32_direct'.
     """
 
-    def __init__(self, model, precision=None, max_batch=16, max_wait_ms=2.0):
+    def __init__(self, model, precision=None, max_batch=16, max_wait_ms=2.0, resize="host"):
         import torch
+        if resize not in ("host", "device"):
+            raise ValueError("resize must be 'host' or 'device' (got %r)" % (resize,))
         self._torch = torch
         self.model = model
         self.precision = precision or getattr(model, "precision", "bf16")
+        self.resize = resize
         self.engine = model.engine()
-        self.batcher = RequestBatcher(self._run_batch, max_batch=max_batch, max_wait_ms=max_wait_ms)
+        run = self._run_batch_device if resize == "device" else self._run_batch
+        self.batcher = RequestBatcher(run, max_batch=max_batch, max_wait_ms=max_wait_ms)
 
     def close(self):
         self.batcher.close()
@@ -142,15 +147,41 @@ class DemoProcessor:
         rgb = bgr.cpu().numpy()[..., ::-1]                                                     # demo.py keeps RGB (test.py swaps to BGR)
         return [np.ascontiguousarray(rgb[i]) for i in range(len(payloads))]
 
+    def _run_batch_device(self, key, payloads):
+        """payloads: (raw RGB image [h,w,3], raw 'L' mask [h',w']) of any raw sizes that floor to ``key``. One copy in, the three
+        resizes of demo.py:45,49,68 and the forward on the device, one copy out."""
+        torch, eng = self._torch, self.engine
+        B = len(payloads)
+        arrays = [p[0] for p in payloads] + [p[1] for p in payloads]
+        offsets = np.concatenate([[0], np.cumsum([a.nbytes for a in arrays])])
+        host = torch.empty(int(offsets[-1]), dtype=torch.uint8, pin_memory=eng.device.type == "cuda")
+        flat = host.numpy()
+        for a, o in zip(arrays, offsets):
+            flat[o:o + a.nbytes] = a.reshape(-1)
+        raw = host.to(eng.device, non_blocking=True)
+        raw_hw = [a.shape[:2] for a in arrays]
+        img = eng.resize_u8(raw, [key] * B, src_hw=raw_hw[:B], channels=3, src_offsets=offsets[:B]).view(B, *key, 3)
+        msk = eng.resize_u8(raw, [key] * B, src_hw=raw_hw[B:], channels=1, src_offsets=offsets[B:2 * B]).view(B, *key)
+        with torch.no_grad():
+            bgr, _ = eng.inference_u8(img, msk, precision=self.precision)
+        rgb = eng.resize_u8(bgr, raw_hw[:B], src_hw=[key] * B, channels=3, reverse_channels=True).cpu().numpy()
+        ends = np.cumsum([h * w * 3 for h, w in raw_hw[:B]])
+        return [rgb[e - h * w * 3:e].reshape(h, w, 3) for e, (h, w) in zip(ends, raw_hw[:B])]
+
     def process_image(self, img, mask):
         """img: PIL image; mask: PIL 'L' image of the same size (non-zero = sketch stroke). Returns the edited PIL image at the
-        input's size. Sizes are floored to a multiple of 8 for the network exactly like demo.py:43."""
+        input's size. Sizes are floored to a multiple of 8 for the network exactly like demo.py:43. With resize='device' the
+        mask must be mode 'L' (Pillow resizes some other modes with another filter); its size may differ from the image's."""
         from PIL import Image
         img = img.convert("RGB")
         w_raw, h_raw = img.size
         h_t, w_t = floor8(h_raw), floor8(w_raw)
         if h_t < 16 or w_t < 16:
             raise ValueError("image smaller than 16x16 (two stride-2 convolutions, 4x4 mask pool, stride-2 patch grid)")
+        if self.resize == "device":
+            if mask.mode != "L":
+                raise ValueError("resize='device' needs an 'L' mask (got mode %r)" % mask.mode)
+            return Image.fromarray(self.batcher.submit((h_t, w_t), (np.asarray(img), np.asarray(mask))))
         img_t = np.ascontiguousarray(np.array(img.resize((w_t, h_t))), dtype=np.uint8)
         mask_t = np.array(mask.resize((w_t, h_t)))
         mask_t = np.ascontiguousarray((mask_t > 0).astype(np.uint8) * 255)
