@@ -110,13 +110,13 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   // has four tile-times per tile); wider tiles keep 2 stages and split a tile's columns between the groups.
   // N <= 64 even fits 8 stages, two per group: while a group drains tile i the MMAs of tile i+4 already fill its second
   // stage, so a group's cycle is the drain alone instead of drain + MMA latency (the small-N layers are epilogue bound)
-  // (the launcher picks the ring sizes: powers of two, or 6 / 3 when three MMA issuer warps share the work - see c8_launch)
+  // (the launcher picks the ring sizes, all powers of two - see c8_launch)
   const int acc_stages = p.acc_stages, acc_stride = p.acc_stride;
   const int epi_split = p.epi_split;
-  // slot / phase parity of iteration i in a ring of n slots (shift = log2 n, or < 0: n is not a power of two)
+  // slot / phase parity of iteration i in a ring of n = 2^shift slots
   auto ring_of = [](int i, int n, int shift, int& slot, uint32_t& phase) {
-    if (shift >= 0) { slot = i & (n - 1); phase = (uint32_t)(i >> shift) & 1u; }
-    else { const int qd = i / n; slot = i - qd * n; phase = (uint32_t)qd & 1u; }
+    slot = i & (n - 1);
+    phase = (uint32_t)(i >> shift) & 1u;
   };
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(wres_bar + 1);
   float* bias_s = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_ptr_smem + 4) + 15) & ~uintptr_t(15));   // 16 B aligned: read with ld.shared.v4
@@ -234,7 +234,7 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
     }
     if (p.dbg && lane == 0) { p.dbg[blockIdx.x * 8 + 0] = t_wait; p.dbg[blockIdx.x * 8 + 1] = clock64() - t_begin; }
-  } else if ((warp == 1 || ((warp == 3 || warp == 2) && !staged)) && (!kPair || cta_rank == 0)) {
+  } else if ((warp == 1 || (warp == 3 && !staged)) && (!kPair || cta_rank == 0)) {
     // ==================================================================== MMA issuer (pair: the leader, for both CTAs)
     // Nothing streamed per k-step (resident weights + halo): a tile is ONE short burst of MMAs, and the issuer's
     // per-tile protocol (two commits, two barrier waits, fence, descriptor set-up: ~600 cycles measured) is longer
@@ -242,9 +242,9 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // between tiles. Warps 1 and 3 therefore issue alternate tiles: each one's protocol overlaps the other's burst.
     // The issuer count must divide every ring it indexes (TMEM stages, halo buffers): a ring slot is then always
     // handled by the same warp, in order - with slots shared between issuers a warp could test a barrier two phases
-    // ahead, and mbarrier parity waits alias modulo 2 (a 3-issuer experiment corrupted tiles and hung exactly so).
+    // ahead, and mbarrier parity waits alias modulo 2.
     auto run_issuer = [&](auto ME_) {
-      const int n_issuers = staged ? 1 : p.niss;   // warps 1, 3, 2 (in this order); the launcher makes both rings multiples of it
+      const int n_issuers = staged ? 1 : p.niss;   // warps 1, 3 (in this order); the launcher makes both rings multiples of it
       // `me` (which of the two issuers this warp is; a second issuer that is not needed simply finds no tile below) is a
       // COMPILE-TIME constant of each copy of this code: everything the MMA operands depend on (tile index, halo buffer, TMEM
       // stage) then derives from blockIdx / parameters / loop counters only, so ptxas keeps the descriptor arithmetic on the
@@ -265,7 +265,7 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // ------------------------------------------------ fused deconv classes (the launcher guarantees two issuers)
         constexpr int CSH = NCLS == 4 ? 2 : 1;
         const int my_tiles = ((int)blockIdx.x < total_tiles) ? (total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-        const int nv = me < 2 ? my_tiles * NCLS : 0;   // two issuers (the classes alternate by parity)
+        const int nv = my_tiles * NCLS;   // two issuers (the classes alternate by parity)
         const uint32_t a_lo = ((p.lbo_bytes >> 4) & 0x3FFF) << 16;
         const uint32_t a_hi = ((p.sbo_bytes >> 4) & 0x3FFF) | (1u << 14);
         const uint32_t b_hi128 = (1024u >> 4) | (1u << 14) | (2u << 29), b_hi64 = (512u >> 4) | (1u << 14) | (4u << 29);
@@ -416,8 +416,7 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       if (p.dbg && lane == 0 && me == 0) { p.dbg[blockIdx.x * 8 + 2] = t_wfull; p.dbg[blockIdx.x * 8 + 3] = t_wtmem; p.dbg[blockIdx.x * 8 + 4] = clock64() - t_begin; p.dbg[blockIdx.x * 8 + 7] = t_whalo; }
     };
     if (warp == 1) run_issuer(std::integral_constant<int, 0>{});
-    else if (warp == 3) run_issuer(std::integral_constant<int, 1>{});
-    else run_issuer(std::integral_constant<int, 2>{});
+    else run_issuer(std::integral_constant<int, 1>{});
   } else if (warp >= 4) {
     // ==================================================================== epilogue
     const int q = warp & 3;
@@ -428,9 +427,8 @@ conv_c8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     long long t_wacc = 0, t_begin = clock64();
     // tile-alternating groups (epi_split == 1) visit every TC_EPI_GROUPS-th tile of this CTA; a tile's coordinates
     // come from two unsigned divisions (cheaper than stepping the mixed-radix counter through the skipped tiles)
-    // Epilogue groups work in TEAMS of epi_split groups: a team drains one tile together (its groups take alternate column blocks),
-    // the TC_EPI_GROUPS / epi_split teams take alternate tiles. epi_split = 1: four one-group teams (N <= 128: one or two TMEM
-    // stages per group); 4: one team (N = 192, two stages); 2: two teams (experiment, see the launcher).
+    // epi_split = 1 (N <= 128): the groups take alternate tiles, one or two TMEM stages each; epi_split = TC_EPI_GROUPS
+    // (N = 192, two stages): all groups drain every tile together, group `sub` taking every epi_split-th column block
     const int nteams = TC_EPI_GROUPS / epi_split, team = grp / epi_split, sub = grp - team * epi_split;
     const int istep = nteams;
     const uint32_t tpi = (uint32_t)(p.tiles_x * p.tiles_y);
@@ -821,59 +819,38 @@ int c8_launch(const ConvParams& c, const C8Layer& L_in, cudaStream_t stream, con
   const int b_bytes = pair ? tc_stage_b_bytes(w) / 2 : tc_stage_b_bytes(w);   // per CTA
   const int stage_bytes = (L.mode == C8_HALO ? 0 : L.a_bytes) + (L.resident ? 0 : b_bytes);
   int fixed = (L.resident ? p.wres_bytes : 0);
-  // ---- rings and MMA issuers. Powers of two by default; a resident layer with nothing streamed per k-step (one short burst
-  // of small-N MMAs per tile) is bound by the ISSUE side - every UTCHMMA operand reaches the uniform registers through R2UR
-  // moves, ~130 cycles per MMA per issuing warp against 40-56 cycles of pipe time (ncu: tensor pipe 35 % active on the
-  // stems with two issuers) - so it gets THREE issuer warps (1, 3 and, after its allocation duty, the TMEM warp 2) and rings of
-  // 6 / 3 slots (an issuer count must divide every ring it indexes: a slot is then always handled by the same warp, in order)
-  // (three issuers need rings of 3 / 6 slots, which the FOUR tile-alternating epilogue groups do not divide: a TMEM stage is then
-  //  drained by changing groups and a group can test its full-barrier a whole phase early - parity waits alias modulo 2 - so this
-  //  stays an experiment switch, default two issuers)
-  static const int niss_cap = getenv("SE_C8_NISS") ? atoi(getenv("SE_C8_NISS")) : 2;
+  // ---- rings and MMA issuers. Every ring is a power of two (the kernel indexes them with a mask and a shift). A resident layer
+  // with nothing streamed per k-step issues one short burst of MMAs per tile, so two issuer warps (1 and 3) take alternate tiles
+  // when its halo ring is even: an issuer count must divide every ring it indexes, so that a slot is always handled by the same
+  // warp, in order
   p.a_bufs = 2;
   p.niss = 1;
   p.acc_stages = w.NT <= 64 ? 8 : (w.NT <= 128 ? 4 : 2);
-  // groups per tile (teams, see the epilogue loop). Two-group teams for 64 < N <= 128 measured SLOWER than one group per tile (stem
-  // pair 916 -> 1040-1096 us, 48->96 787 -> 809-818 us per step at the bench shape): SE_C8_TEAMS=1 is an experiment switch only.
-  static const bool teams_on = getenv("SE_C8_TEAMS") != nullptr && atoi(getenv("SE_C8_TEAMS")) != 0;
-  p.epi_split = w.NT <= 64 ? 1 : (w.NT <= 128 ? ((teams_on && !grp) ? 2 : 1) : TC_EPI_GROUPS);
+  p.acc_stride = w.NT <= 64 ? 64 : (w.NT <= 128 ? 128 : 256);
+  // groups per tile (see the epilogue loop): one for N <= 128, all of them for wider tiles
+  p.epi_split = w.NT <= 128 ? 1 : TC_EPI_GROUPS;
+  SE_REQUIRE(p.epi_split == 1 || c.f16x2 || c.epi == EPI_LINEAR || !epi_fast_ok(p.e) || (c.Cout / 2 + 7) / 8 == 3 * p.epi_split,
+             "a column-split fast gated epilogue needs three 8-column blocks per group");
   if (L.mode == C8_HALO) {
     if (fixed + 2 * L.a_bytes + 3 * stage_bytes > smem_budget) p.a_bufs = 1;   // measured: 2 halo buffers + 3 weight stages beats 1 + 4
     // nothing streamed: a tile is short (700-2000 cycles of MMAs) against a TMA round trip of ~1500 cycles, so two
     // halo buffers leave the tensor pipe waiting for loads; ring as deep as shared memory allows
     if (stage_bytes == 0) {
-      if (!grp && !pair && niss_cap >= 3 && w.NT <= 128 && fixed + 3 * L.a_bytes <= smem_budget) {
-        p.niss = 3;
-        p.a_bufs = (fixed + 6 * L.a_bytes <= smem_budget) ? 6 : 3;
-        p.acc_stages = w.NT <= 64 ? 6 : 3;
-      } else {
-        while (p.a_bufs < C8_MAX_ABUFS && fixed + 2 * p.a_bufs * L.a_bytes <= smem_budget) p.a_bufs *= 2;
-        p.niss = (p.a_bufs % 2 == 0 && niss_cap >= 2) ? 2 : 1;
-      }
+      while (p.a_bufs < C8_MAX_ABUFS && fixed + 2 * p.a_bufs * L.a_bytes <= smem_budget) p.a_bufs *= 2;
+      p.niss = p.a_bufs % 2 == 0 ? 2 : 1;
     }
     fixed += p.a_bufs * L.a_bytes;
-  }
-  p.acc_stride = w.NT <= 64 ? 64 : (w.NT <= 128 ? 128 : 256);
-  // N = 96 resident layers (stem pairs, 48->96, 24->96): four 128-column stages are one per epilogue group, so a group's cycle is
-  // drain (4000-5000 cycles) + refill (TMA wait + MMAs + completion, ~2400) with nothing overlapped (tile timelines, DESIGN.md 5.6).
-  // FIVE stages of 96 columns rotate one spare stage through the four groups: the tile a group takes next is already being
-  // filled while it drains. Stage ownership is then shared, which is only safe with ONE in-order issuer (se_conv_c8.cu header).
-  static const bool five_on = getenv("SE_C8_FIVE") != nullptr && atoi(getenv("SE_C8_FIVE")) != 0;
-  if (five_on && !grp && !pair && stage_bytes == 0 && L.mode == C8_HALO && w.NT == 96 && p.epi_split == 1) {
-    p.acc_stages = 5;
-    p.acc_stride = 96;
-    p.niss = 1;
   }
   p.a_shift = -1;
   for (int sh = 0; sh < 4; ++sh) if ((1 << sh) == p.a_bufs) p.a_shift = sh;
   p.acc_shift = -1;
   for (int sh = 0; sh < 4; ++sh) if ((1 << sh) == p.acc_stages) p.acc_shift = sh;
-  SE_REQUIRE(p.acc_stages * p.acc_stride <= TC_TMEM_COLS && p.a_bufs <= C8_MAX_ABUFS && p.a_bufs % p.niss == 0 && p.acc_stages % p.niss == 0,
+  SE_REQUIRE(p.a_shift >= 0 && p.acc_shift >= 0 && p.acc_stages * p.acc_stride <= TC_TMEM_COLS && p.a_bufs <= C8_MAX_ABUFS &&
+                 p.a_bufs % p.niss == 0 && p.acc_stages % p.niss == 0,
              "ring / issuer plan");
   SE_REQUIRE(!grp || (p.a_bufs >= 2 && w.NT <= 128 && p.ksteps == 1), "fused classes need two halo buffers, <= 128 accumulator columns and a single k-step");
   int stages = stage_bytes ? (smem_budget - fixed) / stage_bytes : 1;
   if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
-  { const char* cap = getenv("SE_C8_STAGES"); if (cap && atoi(cap) >= 2 && atoi(cap) < stages) stages = atoi(cap); }   // experiments
   SE_REQUIRE(stages >= (stage_bytes ? 2 : 1), "shared memory plan does not fit");
   p.num_stages = stages;
   const int smem_bytes = 1024 + fixed + stages * stage_bytes + (2 * TC_MAX_STAGES + 2 * C8_MAX_ABUFS + 17) * 8 + 16 + 3 * (p.NT + 32) * 4 + 64;

@@ -49,10 +49,10 @@ struct C8Params {
   int n64, n32, r64, r32, NT, ksteps;
   const uint8_t* w;
   int mode, HR, WR, pad_y0, pad_x0, cb_in, x_cb_off;
-  int a_bytes, a_tx_bytes, a_bufs, a_shift;   // halo ring: a_bufs buffers; a_shift = log2(a_bufs) or -1 (ring of 3 / 6: index by division)
+  int a_bytes, a_tx_bytes, a_bufs, a_shift;   // halo ring: a_bufs buffers (a power of two), a_shift = log2(a_bufs)
   int acc_stages, acc_shift, acc_stride;      // TMEM accumulator ring (same convention), columns between stages
   int epi_split;                              // 1: the epilogue groups take alternate tiles; 4: they split the columns of every tile
-  int niss;                                   // MMA issuer warps (1-3); must divide both rings
+  int niss;                                   // MMA issuer warps (1 or 2); must divide both rings
   int lbo_bytes, sbo_bytes, kstep_bytes, mmas64;
   uint32_t aoff[C8_MAX_UNITS];   // byte offset of each K unit's A operand inside the shared-memory region
   int num_stages, resident, wres_bytes;

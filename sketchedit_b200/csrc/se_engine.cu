@@ -1126,15 +1126,7 @@ static int run_netG(Ctx& c, const float* x, const float* x2, const float* mask, 
         // split-half mode: fp32 NHWC in / out of the attention (split-half fp16 GEMMs over explicit patch matrices, se_gemm_split.cu)
         Buf f32 = c.get((size_t)c.B * h * w * 96 * 4), o32 = c.get((size_t)c.B * h * w * 96 * 4);
         CK(split_to_f32(pm.p, (float*)f32.p, c.B, 96, h * w, pm.ld / 2, 0, 1, c.stream));
-        static const bool cuda_core_cam = getenv("SE_SPLIT_CAM_DIRECT") != nullptr;   // A/B: the fp32 CUDA-core attention instead
-        if (cuda_core_cam) {
-          const int saved = c.prec;
-          c.prec = SE_PREC_FP32_EXACT;
-          rc = run_cam(c, nhwc(f32.p, h, w, 96, 96), (const float*)ms.p, o32.p, 96, nullptr, 0);
-          c.prec = saved;
-        } else {
-          rc = run_cam_split(c, (const float*)f32.p, h, w, 96, (const float*)ms.p, (float*)o32.p);
-        }
+        rc = run_cam_split(c, (const float*)f32.p, h, w, 96, (const float*)ms.p, (float*)o32.p);
         if (rc) return rc;
         CK(nhwc_f32_to_split((const float*)o32.p, camo.p, c.B, 96, h * w, 12, 0, c.stream));
         c.put(o32); c.put(f32);
@@ -1596,7 +1588,7 @@ int se_contextual_attention_forward(const float* feat, const float* mask_s, int 
   if (!holder) { holder = new se_model(); holder->finalized = true; }
   // fp32-on-tensor-cores mode: split-half GEMM attention (needs 16 * C to be a multiple of 256 and no attention-map output);
   // everything else of the fp32 modes runs on the fp32 CUDA-core kernels
-  const bool split_cam = precision == SE_PREC_FP32_TC && C % 16 == 0 && attn == nullptr && h % 2 == 0 && w % 2 == 0 && getenv("SE_SPLIT_CAM_DIRECT") == nullptr;
+  const bool split_cam = precision == SE_PREC_FP32_TC && C % 16 == 0 && attn == nullptr && h % 2 == 0 && w % 2 == 0;
   if (precision == SE_PREC_FP32_TC) precision = SE_PREC_FP32_EXACT;
   cudaStream_t st = (cudaStream_t)stream;
   return with_arena(holder, precision, B, st, [&](Ctx& c) -> int {

@@ -388,7 +388,7 @@ __device__ __forceinline__ float gate_one(float f, float ghalf, float b, float b
 // blocks (= one 16 B store); no masking is needed because padding columns hold zero weights and zero bias, so they
 // come out as act(0) * sigmoid(0) = 0, which is exactly what the C8 padding channels must contain.
 // nsplit == 1: this group drains the whole tile (16 columns at a time, 8 for an odd last block);
-// nsplit  > 1: the blocks are dealt to the groups, 16 columns at a time if that divides evenly, else 8.
+// nsplit  > 1: the tile has 3 * nsplit blocks, dealt to the groups 8 columns at a time.
 template <bool kElu>
 __device__ __forceinline__ void tc_epilogue_gated_fast(const EpiParams& e, const float* cst, int cst_n, uint32_t taddr, int img, bool valid,
                                                        int oy, int ox, int grp, int nsplit) {
@@ -450,11 +450,10 @@ __device__ __forceinline__ void tc_epilogue_gated_fast(const EpiParams& e, const
     int b = 0;
     for (; b + 2 <= nb; b += 2) do16(b);
     if (b < nb) do8(b);
-  } else if (nb % (2 * nsplit) == 0) {
-    for (int b = 2 * grp; b < nb; b += 2 * nsplit) do16(b);
-  } else if (nb == 3 * nsplit) {
-    // three 8-column blocks per group (192-column tiles over 4 groups): all six TMEM loads are issued before the
-    // single wait, so their latency (long while the MMAs of the next tile stream accumulators) is paid once, not 3x
+  } else {
+    // three 8-column blocks per group (192-column tiles over 4 groups, nb == 3 * nsplit: c8_launch checks it): all six TMEM
+    // loads are issued before the single wait, so their latency (long while the MMAs of the next tile stream accumulators)
+    // is paid once, not 3x
     float f[3][8], g[3][8];
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
@@ -472,8 +471,6 @@ __device__ __forceinline__ void tc_epilogue_gated_fast(const EpiParams& e, const
             make_uint4(pack_bf16x2(f[j][0], f[j][1]), pack_bf16x2(f[j][2], f[j][3]), pack_bf16x2(f[j][4], f[j][5]), pack_bf16x2(f[j][6], f[j][7]));
       }
     }
-  } else {
-    for (int b = grp; b < nb; b += nsplit) do8(b);
   }
 }
 
