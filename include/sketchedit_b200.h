@@ -78,6 +78,21 @@ int se_forward_inference_packed(se_model* m, const float* image, const float* sk
 int se_forward_inference_u8(se_model* m, const unsigned char* image_u8, const unsigned char* sketch_u8, int B, int H, int W,
                             int precision, unsigned char* bgr_u8, unsigned char* mask_u8, void* stream);
 
+/* ---- region inpaint: the user chooses WHERE the edit happens; netM does not run. At inference the reference never takes this
+ *      branch of generate_fake (models/editline2_model.py:340-352 external-mask case, :362-368), which its checkpoints were trained
+ *      for under --joint_train_inp: mask_inpaint = R, line_inpaint = line_full * R, rm2 = R, netG(x, x, R, R, s*R), then
+ *      composed = fine*R + x*(1-R) (:114, :324).
+ * image [B,3,H,W] in [-1,1], sketch [B,1,H,W], region R [B,1,H,W] (1 = edit here), both used as given. Outputs: composed
+ * [B,3,H,W] (equal to image wherever R = 0); optional (may be NULL) coarse, fine [B,3,H,W]. Model options apply as in
+ * se_forward_inference. */
+int se_forward_inpaint(se_model* m, const float* image, const float* sketch, const float* region, int B, int H, int W, int precision,
+                       float* composed, float* coarse, float* fine, void* stream);
+
+/* Same forward with the codecs of se_forward_inference_u8: image_u8 [B,H,W,3] RGB, sketch_u8 and region_u8 [B,H,W] decoded as
+ * s = sketch_u8 > 0, R = region_u8 > 0; output bgr_u8 [B,H,W,3] ((x+1)/2*255 truncated, HWC, RGB->BGR). */
+int se_forward_inpaint_u8(se_model* m, const unsigned char* image_u8, const unsigned char* sketch_u8, const unsigned char* region_u8,
+                          int B, int H, int W, int precision, unsigned char* bgr_u8, void* stream);
+
 /* ---- netM: replaces MDGenerator.forward(x, guide) -> (mask1, x_stage1)  (editline2_g.py:59-94) */
 int se_netM_forward(se_model* m, const float* x, const float* guide, int B, int H, int W, int precision, float* mask1,
                     float* x_stage1 /* may be NULL */, void* stream);

@@ -3,8 +3,9 @@
 ``forward(data, mode)`` with mode 'inference' returns ``(composed_image, mask)`` exactly like the
 reference: netM predicts the edit mask from (image, sketch), the mask is binarised at 0.5, netG inpaints,
 and the result is blended with the SOFT mask. All of it is one C-ABI call (``se_forward_inference``) on the
-B200 kernels; tensors in ``data`` may live on the CPU (they are copied to the GPU like the reference's
-``preprocess_input`` does) and the outputs are CUDA tensors. Training modes are out of scope."""
+B200 kernels. Mode 'inpaint' takes the region to edit from ``data['region']`` instead of netM and returns
+``(composed_image, region)`` (one ``se_forward_inpaint`` call). In both, tensors in ``data`` may live on the CPU
+(they are copied to the GPU like the reference's ``preprocess_input`` does) and the outputs are CUDA tensors. Training modes are out of scope."""
 import torch
 
 import models.networks as networks
@@ -63,6 +64,7 @@ class EditLine2Model(torch.nn.Module):
         return image, line
 
     def forward(self, data, mode, is_real_im=True):
+        region = data["region"] if mode == "inpaint" else None
         image, line = self.preprocess_input(data)
         if mode == "inference":
             composed, mask, _ = self.engine().inference(image, line, precision=self.precision)
@@ -74,6 +76,12 @@ class EditLine2Model(torch.nn.Module):
                                                       want=("coarse", "fine", "mask_image", "mask_bin"))
             return {"mask": ex["mask_bin"], "maskim": ex["mask_image"], "coarse": ex["coarse"], "fine": ex["fine"],
                     "composed": composed}
+        if mode == "inpaint":
+            # the user chooses the region (data['region'] [B,1,H,W], 1 = edit here) instead of netM: the external-mask branch of the
+            # reference's generate_fake (:340-352, 362-368) composed like :114. Returns (composed, region) like 'inference' does.
+            region = region.to(image.device, torch.float32, non_blocking=True)
+            composed, _ = self.engine().inpaint(image, line, region, precision=self.precision)
+            return composed, region
         raise ValueError("|mode| is invalid or training-only: %r" % (mode,))
 
     def inference_stream(self, loader, depth=2, pinned_ring=True, gather=None, uint8=False, with_data=False):

@@ -30,6 +30,9 @@ SIGNATURES = {
                                       _c_void_p]),
     "se_forward_inference_packed": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_void_p, _c_void_p]),
     "se_forward_inference_u8": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_void_p, _c_void_p, _c_void_p]),
+    "se_forward_inpaint": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_void_p, _c_void_p,
+                                    _c_void_p, _c_void_p]),
+    "se_forward_inpaint_u8": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_void_p, _c_void_p]),
     "se_netM_forward": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_void_p, _c_void_p,
                                  _c_void_p]),
     "se_netG_forward": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int,

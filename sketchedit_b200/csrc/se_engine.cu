@@ -1488,6 +1488,46 @@ int se_forward_inference_u8(se_model* m, const unsigned char* image_u8, const un
   }, key);
 }
 
+// generate_fake's external-mask branch at inference (editline2_model.py:343-345,362-368): netG(x, x, R, R, s*R), composed with R
+// (:114); netM does not run. The final head's blend with R in place of the soft mask leaves x bit for bit where R = 0.
+int se_forward_inpaint(se_model* m, const float* image, const float* sketch, const float* region, int B, int H, int W, int precision,
+                       float* composed, float* coarse, float* fine, void* stream) {
+  SE_REQUIRE(image && sketch && region && composed, "null tensor");
+  int rc = check_hw(H, W);
+  if (rc) return rc;
+  std::vector<uintptr_t> key = {5, (uintptr_t)H, (uintptr_t)W, (uintptr_t)image, (uintptr_t)sketch, (uintptr_t)region, (uintptr_t)composed,
+                                (uintptr_t)coarse, (uintptr_t)fine};
+  return with_arena(m, precision, B, (cudaStream_t)stream, [&](Ctx& c) -> int {
+    Buf sr = c.get((size_t)B * H * W * 4);
+    c.tag("region_inputs_kernel|sketch * region", 0, 0, 0, (double)B * H * W * 12);
+    CK(region_sketch(sketch, region, (float*)sr.p, B, H, W, c.stream));
+    int r = run_netG(c, image, image, region, region, (const float*)sr.p, H, W, coarse, fine, composed, region, image);
+    if (r) return r;
+    c.put(sr);
+    return 0;
+  }, key);
+}
+
+int se_forward_inpaint_u8(se_model* m, const unsigned char* image_u8, const unsigned char* sketch_u8, const unsigned char* region_u8, int B, int H,
+                          int W, int precision, unsigned char* bgr_u8, void* stream) {
+  SE_REQUIRE(image_u8 && sketch_u8 && region_u8 && bgr_u8, "null tensor");
+  int rc = check_hw(H, W);
+  if (rc) return rc;
+  std::vector<uintptr_t> key = {6, (uintptr_t)H, (uintptr_t)W, (uintptr_t)image_u8, (uintptr_t)sketch_u8, (uintptr_t)region_u8, (uintptr_t)bgr_u8};
+  return with_arena(m, precision, B, (cudaStream_t)stream, [&](Ctx& c) -> int {
+    // input codec (the sketch's, data/testimage_dataset.py:89-103, also for the region) -> netG -> output codec fused into the last head
+    Buf img = c.get((size_t)B * 3 * H * W * 4), rg = c.get((size_t)B * H * W * 4), sr = c.get((size_t)B * H * W * 4);
+    c.tag("region_inputs_kernel|input codec + sketch * region", 0, 0, 0, (double)B * H * W * (5 + 20));
+    CK(region_inputs_u8(image_u8, sketch_u8, region_u8, (float*)img.p, (float*)rg.p, (float*)sr.p, B, H, W, c.stream));
+    const float* x = (const float*)img.p;
+    const float* R = (const float*)rg.p;
+    int r = run_netG(c, x, x, R, R, (const float*)sr.p, H, W, nullptr, nullptr, nullptr, R, x, 0, 0, bgr_u8);
+    if (r) return r;
+    c.put(sr); c.put(rg); c.put(img);
+    return 0;
+  }, key);
+}
+
 int se_netM_forward(se_model* m, const float* x, const float* guide, int B, int H, int W, int precision, float* mask1, float* x_stage1,
                     void* stream) {
   SE_REQUIRE(x && guide && mask1, "null tensor");

@@ -795,6 +795,39 @@ int u8_to_inputs(const unsigned char* img_u8, const unsigned char* sk_u8, float*
   return 0;
 }
 
+// inputs of the region inpaint (reference editline2_model.py:343-345: line_inpaint = line_full * mask_inpaint): uint8 entry
+// (T = unsigned char): image HWC RGB -> fp32 NCHW as u8_to_inputs_kernel, R = region > 0, s*R with s = sketch > 0; float entry
+// (T = float, img_u8 and region NULL): only s*R from the caller's planes
+__device__ __forceinline__ float region_plane(unsigned char v) { return v > 0 ? 1.0f : 0.0f; }
+__device__ __forceinline__ float region_plane(float v) { return v; }
+template <typename T>
+__global__ void region_inputs_kernel(const unsigned char* __restrict__ img_u8, const T* __restrict__ sk_in, const T* __restrict__ rg_in,
+                                     float* __restrict__ img, float* __restrict__ region, float* __restrict__ sk_region, int B, long long HW) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= B * HW) return;
+  if (img_u8) {
+    const long long b = i / HW, pix = i % HW;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) img[(b * 3 + c) * HW + pix] = (__fdiv_rn((float)img_u8[i * 3 + c], 255.0f) - 0.5f) / 0.5f;
+  }
+  const float r = region_plane(rg_in[i]);
+  if (region) region[i] = r;
+  sk_region[i] = region_plane(sk_in[i]) * r;
+}
+int region_inputs_u8(const unsigned char* img_u8, const unsigned char* sk_u8, const unsigned char* rg_u8, float* img, float* region, float* sk_region,
+                     int B, int H, int W, cudaStream_t s) {
+  const long long HW = (long long)H * W;
+  region_inputs_kernel<unsigned char><<<cdiv(B * HW, 256), 256, 0, s>>>(img_u8, sk_u8, rg_u8, img, region, sk_region, B, HW);
+  SE_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+int region_sketch(const float* sketch, const float* region, float* sk_region, int B, int H, int W, cudaStream_t s) {
+  const long long HW = (long long)H * W;
+  region_inputs_kernel<float><<<cdiv(B * HW, 256), 256, 0, s>>>(nullptr, sketch, region, nullptr, nullptr, sk_region, B, HW);
+  SE_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
 // test.py:25-27,33-35: (mask*255).astype(uint8); ((x+1)/2*255).astype(uint8) (truncation), CHW->HWC, RGB->BGR
 __global__ void to_uint8_kernel(const float* __restrict__ comp, const float* __restrict__ mask, unsigned char* __restrict__ bgr,
                                 unsigned char* __restrict__ mk, int B, long long HW) {

@@ -31,6 +31,10 @@ int c8_to_nchw(const void* x, float* y, int B, int C, int HW, cudaStream_t s);
 int nchw_to_nhwc(const float* x, void* y, int dt, int B, int C, int HW, int ldo, int choff, cudaStream_t s);
 int nhwc_to_nchw(const void* x, int dt, float* y, int B, int C, int HW, int ldx, int choff, cudaStream_t s);
 int u8_to_inputs(const unsigned char* img_u8, const unsigned char* sk_u8, float* img, float* sk, int B, int H, int W, cudaStream_t s);
+// region inpaint inputs (one kernel): uint8 entry -> image, R = region > 0 and s*R planes; float entry -> the s*R plane only
+int region_inputs_u8(const unsigned char* img_u8, const unsigned char* sk_u8, const unsigned char* rg_u8, float* img, float* region, float* sk_region,
+                     int B, int H, int W, cudaStream_t s);
+int region_sketch(const float* sketch, const float* region, float* sk_region, int B, int H, int W, cudaStream_t s);
 int to_uint8(const float* comp, const float* mask, unsigned char* bgr, unsigned char* mk, int B, int H, int W, cudaStream_t s);
 // split-half twins (se_split.cu): activations stored as fp16 hi + fp16 lo (DT_F16X2)
 int pack8_split(const float* img, const float* sketch, const float* mask, void* out, int B, int H, int W, int Wp, int padl, int img_mode,

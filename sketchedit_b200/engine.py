@@ -240,6 +240,46 @@ class Engine:
                                                     _stream()))
         return bgr, mk
 
+    def inpaint(self, image, sketch, region, precision="bf16", want=(), out=None):
+        """Edit a region the caller chooses, without netM: ``coarse, fine = netG(image, image, region, region, sketch * region)``
+        and ``composed = fine * region + image * (1 - region)``, which equals ``image`` wherever region is 0. image [B,3,H,W] in
+        [-1,1], sketch and region [B,1,H,W] (region 1 = edit here). Returns (composed, dict of ``want`` among ('coarse', 'fine'));
+        ``out`` is a caller-owned fp32 CUDA tensor [B,3,H,W] for composed."""
+        image = _chk_in(image, name="image")
+        sketch = _chk_in(sketch, name="sketch")
+        region = _chk_in(region, name="region")
+        B, _, H, W = image.shape
+        for t, nm in ((sketch, "sketch"), (region, "region")):
+            if tuple(t.shape) != (B, 1, H, W):
+                raise _lib.SketchEditB200Error("%s must have shape %r (got %r)" % (nm, (B, 1, H, W), tuple(t.shape)))
+        if set(want) - {"coarse", "fine"}:
+            raise _lib.SketchEditB200Error("want may hold 'coarse' and 'fine' (got %r)" % (tuple(want),))
+        composed = _f32(B, 3, H, W, like=image) if out is None else _chk_out(out, (B, 3, H, W), "out")
+        extra = {k: _f32(B, 3, H, W, like=image) for k in want}
+        self._on_device(image, sketch, region, composed)
+        _lib.check(self.lib.se_forward_inpaint(self.h, _ptr(image), _ptr(sketch), _ptr(region), B, H, W, _lib.PREC[precision], _ptr(composed),
+                                               _ptr(extra.get("coarse")), _ptr(extra.get("fine")), _stream()))
+        return composed, extra
+
+    def inpaint_u8(self, image_u8, sketch_u8, region_u8, precision="bf16", out=None):
+        """``inpaint`` with the codecs of ``inference_u8``: image_u8 [B,H,W,3] RGB, sketch_u8 and region_u8 [B,H,W] uint8 (non-zero =
+        stroke / edit here) -> bgr_u8 [B,H,W,3] as test.py:25-35 writes images. ``out`` is a caller-owned uint8 CUDA tensor."""
+        for t, nm in ((image_u8, "image_u8"), (sketch_u8, "sketch_u8"), (region_u8, "region_u8")):
+            _chk_u8(t, nm)
+        B, H, W, C = image_u8.shape
+        if C != 3 or tuple(sketch_u8.shape) != (B, H, W) or tuple(region_u8.shape) != (B, H, W):
+            raise _lib.SketchEditB200Error("image_u8 must be [B,H,W,3], sketch_u8 and region_u8 [B,H,W]")
+        if out is None:
+            bgr = torch.empty(B, H, W, 3, device=image_u8.device, dtype=torch.uint8)
+        elif tuple(_chk_u8(out, "out").shape) != (B, H, W, 3):
+            raise _lib.SketchEditB200Error("out must be a contiguous CUDA uint8 [B,H,W,3] tensor")
+        else:
+            bgr = out
+        self._on_device(image_u8, sketch_u8, region_u8, bgr)
+        _lib.check(self.lib.se_forward_inpaint_u8(self.h, _ptr(image_u8), _ptr(sketch_u8), _ptr(region_u8), B, H, W, _lib.PREC[precision],
+                                                  _ptr(bgr), _stream()))
+        return bgr
+
     # the model-less device resize, next to the forward it brackets in serving (and replaceable there by a test double)
     resize_u8 = staticmethod(resize_u8)
 

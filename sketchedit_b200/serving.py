@@ -138,21 +138,29 @@ class DemoProcessor:
     def close(self):
         self.batcher.close()
 
+    def _forward_u8(self, img, planes):
+        """planes: (sketch,) -> the netM forward; (sketch, region) -> the region inpaint (Engine.inpaint_u8). Returns BGR uint8."""
+        with self._torch.no_grad():
+            if len(planes) == 2:
+                return self.engine.inpaint_u8(img, *planes, precision=self.precision)
+            return self.engine.inference_u8(img, *planes, precision=self.precision)[0]
+
     def _run_batch(self, key, payloads):
-        torch = self._torch
-        img = torch.from_numpy(np.stack([p[0] for p in payloads])).cuda(non_blocking=True)     # [B,H,W,3] RGB uint8
-        msk = torch.from_numpy(np.stack([p[1] for p in payloads])).cuda(non_blocking=True)     # [B,H,W] uint8 (> 0 = stroke)
-        with torch.no_grad():
-            bgr, _ = self.engine.inference_u8(img, msk, precision=self.precision)
-        rgb = bgr.cpu().numpy()[..., ::-1]                                                     # demo.py keeps RGB (test.py swaps to BGR)
+        torch, dev = self._torch, self.engine.device
+        img = torch.from_numpy(np.stack([p[0] for p in payloads])).to(dev, non_blocking=True)           # [B,H,W,3] RGB uint8
+        planes = [torch.from_numpy(np.stack([p[k] for p in payloads])).to(dev, non_blocking=True)        # [B,H,W] uint8 (> 0 = stroke,
+                  for k in range(1, len(payloads[0]))]                                                  # > 0 = edit here)
+        rgb = self._forward_u8(img, planes).cpu().numpy()[..., ::-1]                                    # demo.py keeps RGB (test.py swaps to BGR)
         return [np.ascontiguousarray(rgb[i]) for i in range(len(payloads))]
 
     def _run_batch_device(self, key, payloads):
-        """payloads: (raw RGB image [h,w,3], raw 'L' mask [h',w']) of any raw sizes that floor to ``key``. One copy in, the three
-        resizes of demo.py:45,49,68 and the forward on the device, one copy out."""
+        """payloads: (raw RGB image [h,w,3], raw 'L' mask [h',w'][, raw 'L' region [h'',w'']]) of any raw sizes that floor to
+        ``key``. One copy in, the resizes of demo.py:45,49,68 (the region's like the mask's) and the forward on the device, one copy
+        out."""
         torch, eng = self._torch, self.engine
-        B = len(payloads)
-        arrays = [p[0] for p in payloads] + [p[1] for p in payloads]
+        B, n = len(payloads), len(payloads[0])
+        size = tuple(key[:2])
+        arrays = [p[k] for k in range(n) for p in payloads]              # images, then masks, then regions
         offsets = np.concatenate([[0], np.cumsum([a.nbytes for a in arrays])])
         host = torch.empty(int(offsets[-1]), dtype=torch.uint8, pin_memory=eng.device.type == "cuda")
         flat = host.numpy()
@@ -160,30 +168,36 @@ class DemoProcessor:
             flat[o:o + a.nbytes] = a.reshape(-1)
         raw = host.to(eng.device, non_blocking=True)
         raw_hw = [a.shape[:2] for a in arrays]
-        img = eng.resize_u8(raw, [key] * B, src_hw=raw_hw[:B], channels=3, src_offsets=offsets[:B]).view(B, *key, 3)
-        msk = eng.resize_u8(raw, [key] * B, src_hw=raw_hw[B:], channels=1, src_offsets=offsets[B:2 * B]).view(B, *key)
-        with torch.no_grad():
-            bgr, _ = eng.inference_u8(img, msk, precision=self.precision)
-        rgb = eng.resize_u8(bgr, raw_hw[:B], src_hw=[key] * B, channels=3, reverse_channels=True).cpu().numpy()
+        img = eng.resize_u8(raw, [size] * B, src_hw=raw_hw[:B], channels=3, src_offsets=offsets[:B]).view(B, *size, 3)
+        planes = [eng.resize_u8(raw, [size] * B, src_hw=raw_hw[k * B:(k + 1) * B], channels=1, src_offsets=offsets[k * B:(k + 1) * B]).view(B, *size)
+                  for k in range(1, n)]
+        bgr = self._forward_u8(img, planes)
+        rgb = eng.resize_u8(bgr, raw_hw[:B], src_hw=[size] * B, channels=3, reverse_channels=True).cpu().numpy()
         ends = np.cumsum([h * w * 3 for h, w in raw_hw[:B]])
         return [rgb[e - h * w * 3:e].reshape(h, w, 3) for e, (h, w) in zip(ends, raw_hw[:B])]
 
-    def process_image(self, img, mask):
+    def process_image(self, img, mask, region=None):
         """img: PIL image; mask: PIL 'L' image of the same size (non-zero = sketch stroke). Returns the edited PIL image at the
         input's size. Sizes are floored to a multiple of 8 for the network exactly like demo.py:43. With resize='device' the
-        mask must be mode 'L' (Pillow resizes some other modes with another filter); its size may differ from the image's."""
+        mask must be mode 'L' (Pillow resizes some other modes with another filter); its size may differ from the image's.
+
+        region: None (netM chooses where to edit) or a PIL 'L' image, non-zero = edit here, resized and binarised exactly like the
+        mask. The edit then stays inside it (``Engine.inpaint_u8``); such requests batch apart from plain ones, under
+        ``(h, w, "region")``."""
         from PIL import Image
         img = img.convert("RGB")
         w_raw, h_raw = img.size
         h_t, w_t = floor8(h_raw), floor8(w_raw)
         if h_t < 16 or w_t < 16:
             raise ValueError("image smaller than 16x16 (two stride-2 convolutions, 4x4 mask pool, stride-2 patch grid)")
+        planes = (mask,) if region is None else (mask, region)
+        key = (h_t, w_t) if region is None else (h_t, w_t, "region")
         if self.resize == "device":
-            if mask.mode != "L":
-                raise ValueError("resize='device' needs an 'L' mask (got mode %r)" % mask.mode)
-            return Image.fromarray(self.batcher.submit((h_t, w_t), (np.asarray(img), np.asarray(mask))))
+            for p in planes:
+                if p.mode != "L":
+                    raise ValueError("resize='device' needs 'L' masks and regions (got mode %r)" % p.mode)
+            return Image.fromarray(self.batcher.submit(key, (np.asarray(img),) + tuple(np.asarray(p) for p in planes)))
         img_t = np.ascontiguousarray(np.array(img.resize((w_t, h_t))), dtype=np.uint8)
-        mask_t = np.array(mask.resize((w_t, h_t)))
-        mask_t = np.ascontiguousarray((mask_t > 0).astype(np.uint8) * 255)
-        out = self.batcher.submit((h_t, w_t), (img_t, mask_t))
+        planes_t = tuple(np.ascontiguousarray((np.array(p.resize((w_t, h_t))) > 0).astype(np.uint8) * 255) for p in planes)
+        out = self.batcher.submit(key, (img_t,) + planes_t)
         return Image.fromarray(out).resize((w_raw, h_raw))
